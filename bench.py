@@ -57,7 +57,19 @@ def parse_args():
                     help="value-net kernel: tcx2 (default) = tcgen05 fp16 operands with the fast fp32 tanh GELU, tc = the same with the logistic fp32 GELU, fp32 = SIMT parity net")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample", type=int, default=0, help="subgames in the CPU-baseline sample (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="datagen / config4: write the training examples of the last timed wave (rank 0) to DIR/*.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.workload not in ("datagen", "config4"):
+        ap.error("--dump-outputs is implemented for the datagen and config4 workloads")
+    return args
+
+
+def dump_outputs(out_dir, arrays):
+    """One float32 .npy per array: the outputs of two builds run with the same arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, np.float32))
 
 
 def dims(D, F):
@@ -602,13 +614,16 @@ def run_datagen(args):
         if not no_flush:
             S.l2_flush()
         finish_and_start(True, True)
-    finish_and_start(False, True)
+    n_last = finish_and_start(False, True)
     S.mark(1)
     ms = S.elapsed_ms(0, 1)
     barrier()
     if rank == 0:
         sampler.window(t_region0, time.perf_counter())
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:             # the last wave's rows, as appended to the replay rows (query, value target)
+        q, v = S.selfplay_examples()
+        dump_outputs(args.dump_outputs, {"examples_query": q.reshape(-1, Q)[:n_last], "examples_value": v.reshape(-1, H)[:n_last]})
     ms = rbdist.max_over_ranks(ms, dev)
     launches = S.kernel_launches - launches0
     value = world * K * iters * steps / (ms * 1e-3)

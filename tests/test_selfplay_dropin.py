@@ -1,75 +1,88 @@
 """The reference's UNMODIFIED cfvpy/selfplay.py against the rebel_b200 `rela` module (SURVEY 8b: selfplay.py drops in unchanged).
 
-selfplay.py imports hydra-era packages that are not in this image (omegaconf, pytorch_lightning, heyhi's launcher); they are
-stubbed with empty modules — none of them is on the data-generation path — and `cfvpy.rela` resolves to rebel_b200.rela.  Runs only
-where the reference checkout exists (the build container); nothing of it is copied into the repository."""
-import importlib.util
+What selfplay.py does with the module was recorded by running it against rebel_b200.rela (oracle/make_golden_crosscheck.py,
+tests/golden/selfplay_dropin.json): the attribute operations of create_mdp_config, the parameters of the Net2 models
+_build_model builds, their outputs and get_last_action_index on query rows of the C port.  The tests replay those operations
+on the module and compare with the recording; nothing of the reference's code is in the repository."""
+import json
 import os
-import sys
-import types
 
+import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference/cfvpy"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "selfplay_dropin.json")
 
 
 @pytest.fixture(scope="module")
 def selfplay():
-    import rebel_b200.rela as rela
-    saved = {k: sys.modules.get(k) for k in ("cfvpy", "cfvpy.rela", "cfvpy.models", "cfvpy.utils", "cfvpy.selfplay", "heyhi", "omegaconf",
-                                             "omegaconf.dictconfig", "pytorch_lightning", "pytorch_lightning.logging")}
-    pkg = types.ModuleType("cfvpy"); pkg.__path__ = [REF]
-    heyhi = types.ModuleType("heyhi"); heyhi.is_on_slurm = lambda: False
-    oc = types.ModuleType("omegaconf"); ocd = types.ModuleType("omegaconf.dictconfig")
-    ocd.DictConfig = type("DictConfig", (dict,), {}); oc.dictconfig = ocd
-    pl = types.ModuleType("pytorch_lightning"); pll = types.ModuleType("pytorch_lightning.logging"); pl.logging = pll
-    sys.modules.update({"cfvpy": pkg, "cfvpy.rela": rela, "heyhi": heyhi, "omegaconf": oc, "omegaconf.dictconfig": ocd,
-                        "pytorch_lightning": pl, "pytorch_lightning.logging": pll})
-    pkg.rela = rela
-    spec = importlib.util.spec_from_file_location("cfvpy.selfplay", os.path.join(REF, "selfplay.py"))
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules["cfvpy.selfplay"] = mod
-    spec.loader.exec_module(mod)
-    yield mod
-    for k, v in saved.items():
-        if v is None:
-            sys.modules.pop(k, None)
-        else:
-            sys.modules[k] = v
+    with open(GOLDEN) as f:
+        return json.load(f)
+
+
+def _replay_mdp_config(rela, case):
+    """create_mdp_config (selfplay.py:587-610) as recorded: hasattr before every key, getattr to recurse into subgame_params,
+    setattr of every leaf value; it raises when hasattr is false."""
+    cfg = rela.RecursiveSolvingParams()
+
+    def parent(path):
+        obj = cfg
+        for name in path.split(".")[:-1]:
+            obj = getattr(obj, name)
+        return obj, path.split(".")[-1]
+    for op, path, value in case["ops"]:
+        obj, name = parent(path)
+        assert hasattr(obj, name) == (op != "missing"), (op, path)
+        if op == "set":
+            setattr(obj, name, value)
+    if case["raised"]:
+        assert case["ops"][-1][0] == "missing"
+    return cfg
 
 
 def test_create_mdp_config_fills_our_params(selfplay):
     """create_mdp_config (selfplay.py:587-610): hasattr / setattr over cfg.env, recursing into subgame_params; B200 knobs are
     ordinary extra keys; unknown keys raise like with the reference module."""
     import rebel_b200.rela as rela
-    env = {"num_dice": 1, "num_faces": 6, "random_action_prob": 0.25, "sample_leaf": True,
-           "subgame_params": {"num_iters": 1024, "max_depth": 2, "linear_update": True, "use_cfr": True},
-           "concurrent_games": 4096, "net_mode": 3}
-    cfg = selfplay.create_mdp_config(env)
+    full, unknown, empty = selfplay["create_mdp_config"]
+    assert full["raised"] is None and len(full["ops"]) == 22
+    cfg = _replay_mdp_config(rela, full)
     assert isinstance(cfg, rela.RecursiveSolvingParams)
     assert (cfg.num_dice, cfg.num_faces, cfg.sample_leaf, cfg.concurrent_games) == (1, 6, True, 4096)
     assert abs(cfg.random_action_prob - 0.25) < 1e-7
     sp = cfg.subgame_params
     assert (sp.num_iters, sp.max_depth, sp.linear_update, sp.use_cfr) == (1024, 2, True, True)
-    with pytest.raises(RuntimeError, match="Cannot find key"):
-        selfplay.create_mdp_config({"no_such_knob": 1})
-    assert isinstance(selfplay.create_mdp_config(None), rela.RecursiveSolvingParams)
+    assert unknown["env"] == {"no_such_knob": 1} and unknown["raised"] == "Cannot find key no_such_knob"
+    _replay_mdp_config(rela, unknown)
+    assert empty["env"] is None and empty["ops"] == [] and empty["raised"] is None
+    assert isinstance(_replay_mdp_config(rela, empty), rela.RecursiveSolvingParams)
 
 
-def test_reference_model_builder_feeds_our_model_locker(selfplay):
+def test_reference_model_builder_feeds_our_model_locker(selfplay, port):
     """_build_model (selfplay.py:31-50) with the YAML's model block (liars_sp.yaml:28-33) produces the TorchScript Net2 our
     ModelLocker accepts; the reference's default Net2 (n_layers=3) is refused instead of being truncated."""
     import rebel_b200.rela as rela
-    ns = types.SimpleNamespace
-    env = ns(num_faces=6, num_dice=1)
-    good = selfplay._build_model("cpu", env, ns(name="Net2", kwargs=dict(n_hidden=256, use_layer_norm=True, n_layers=2)), jit=True)
+    from oracle.make_golden_crosscheck import DROPIN_LAST_BIDS, dropin_query_rows
+    from rebel_b200.models import Net2, make_selfplay_net
+    models = selfplay["models"]
+    built = {}
+    for name, rec in models.items():
+        net = Net2(num_faces=6, num_dice=1, **rec["kwargs"])
+        assert [[k, list(v.shape)] for k, v in net.state_dict().items()] == rec["parameters"], name
+        built[name] = net
+    built["yaml"].load_state_dict(make_selfplay_net(1, 6, seed=0).state_dict())
+    good = torch.jit.script(built["yaml"])
     locker = rela.ModelLocker([good], "cuda:0")
     assert locker.version == 1
-    q = torch.zeros(4, 2 + 13 + 12)
-    assert good(q).shape == (4, 6)
-    assert torch.equal(selfplay.get_last_action_index(q, 13), torch.full((4,), 13))      # all-zero one-hot = "initial"
-    deep = selfplay._build_model("cpu", env, ns(name="Net2", kwargs=dict(n_hidden=256, use_layer_norm=True)), jit=True)
+    rows = dropin_query_rows(port)
+    assert np.array_equal(rows, np.asarray(selfplay["query_rows"], np.float32))
+    with torch.no_grad():
+        out = good(torch.from_numpy(rows)).numpy()
+    assert out.shape == (len(rows), 6)
+    assert np.allclose(out, np.asarray(selfplay["yaml_model_outputs_seed0"], np.float32), rtol=1e-5, atol=1e-7)
+    # the last bid of our query rows, as the reference's get_last_action_index decodes it: 13 = "initial" (all-zero one-hot)
+    A = 13
+    assert selfplay["get_last_action_index"] == [A] + [A if lb < 0 else lb for lb in DROPIN_LAST_BIDS for _ in (0, 1)]
+    deep = torch.jit.script(built["default_layers"])
     with pytest.raises(RuntimeError, match="unexpected parameter"):
         rela.ModelLocker([deep], "cuda:0")
