@@ -64,9 +64,7 @@ enum {
   CFRB_NET_TC_F16 = 2,    /* tcgen05 tensor-core kernel: fp16 operands, fp32 accumulate/LayerNorm/GELU
                              (the reference's own `half_inference` option, selfplay.py:42-43,211) */
   CFRB_NET_TC_F16X2 = 3   /* same kernel with the fast GELU: y/2 (1 + tanh(poly)) with packed f32x2 FMAs and tanh.approx.f32, one
-                             rounding to fp16 at the end (same accuracy as mode 2, 1 instead of 2 MUFU operations per element).
-                             CFRB_X2_GELU=half selects the packed-fp16 evaluation (HFMA2 + tanh.approx.f16x2): 6 % faster, but
-                             that instruction truncates towards zero and biases every activation (see DESIGN.md "P5") */
+                             rounding to fp16 at the end (same accuracy as mode 2, 1 instead of 2 MUFU operations per element) */
 };
 
 /* Subgame solver.  In FP mode cfrb_fetch's "last" is FP::last_strategies (belief x best response), "avg" is
@@ -189,7 +187,7 @@ int cfrb_debug_leaf_io(cfrb_handle* h, float* queries, float* net_out, double* s
  * the raw fp32 accumulators of layer 1 and layer 2 for the first 128 rows, each [128][256]. */
 int cfrb_debug_net_taps(cfrb_handle* h, float* d1, float* d2);
 /* Development aid: re-runs the tensor-core value net once with clock64() stamps of CTA 0 (out[2048]: epilogue thread 0 at
- * [iter*16 + e], MMA-issuing thread at [1024 + iter*8 + m]; see leaf_mlp_tc.cuh). */
+ * [phase*8 + e], MMA-issuing thread at [1024 + phase*4 + m]; see the CFRB_TRACE3 calls in leaf_mlp_tc3.cuh). */
 int cfrb_debug_net_trace(cfrb_handle* h, long long* out, int n);
 
 /* Exploitability (best-response values of both players, compute_exploitability2) of a full-tree strategy
@@ -229,11 +227,12 @@ int cfrb_selfplay_wait_examples(cfrb_handle* h);
 /* Game states (public state and beliefs [n][2][H]) copied to the host; any pointer may be NULL.  Synchronises.  Returns n_games. */
 int cfrb_selfplay_state(cfrb_handle* h, int32_t* last_bid, int32_t* player, double* beliefs);
 /* Test aid: the division-free quotient of the regret-matching step (reciprocal of the node's sum + two fused multiply-add
- * corrections, csrc/cfr_d2v2.cuh) against IEEE division on blocks x 256 x 4096 pseudo-random operand pairs. */
+ * corrections, csrc/cfr_kernels.cuh) against IEEE division on blocks x 256 x 4096 pseudo-random operand pairs. */
 int cfrb_debug_div_check(cfrb_handle* h, uint64_t seed, int32_t blocks, uint64_t* mismatches);
-/* Test aid: the packed-half GELU of the value-net epilogue on every fp16 input: out[i] = fp16 bits of f(fp16 with bit pattern i), i < 65536;
- * what 0 = tanh.approx.f16x2, 1 / 2 = GELU(2 x) computed from x = y / 2 the way the packed-half / fp32-tanh epilogue does (tests pin the arithmetic model of
- * oracle/ref_harness.cc against it). */
+/* Test aid: GELU evaluations on every fp16 input: out[i] = fp16 bits of f(fp16 with bit pattern i), i < 65536;
+ * what 0 = tanh.approx.f16x2, 1 / 2 = GELU(2 x) computed from x = y / 2 in packed-half arithmetic (HFMA2 + tanh.approx.f16x2, a
+ * biased evaluation the value net does not use) / the way the fp32-tanh epilogue of CFRB_NET_TC_F16X2 does (tests pin the
+ * arithmetic model of oracle/ref_harness.cc against it). */
 int cfrb_debug_gelu_table(cfrb_handle* h, int32_t what, uint16_t* out);
 /* Roots (last_bid, player_id) of the subgames of the current wave — also of a wave built on the device by cfrb_selfplay_wave
  * (synchronises then).  Writes min(n, cap) entries, returns n. */

@@ -6,7 +6,6 @@
 #include "cfr_kernels.cuh"
 #include "br_kernel.cuh"
 #include "selfplay_kernels.cuh"
-#include "cfr_d2v2.cuh"
 
 namespace cfrb {
 
@@ -111,33 +110,6 @@ void rows_launch_gather(const float* src, int width, const int* ids, int n, floa
   rows_gather_kernel<<<blocks, 256, 0, st>>>(src, width, ids, n, out);
 }
 
-template <typename real>
-cudaError_t cfr_configure_d2v2(int smem_bytes) {
-  cudaError_t e = cudaSuccess;
-#define CFRB_CFG1(HC, GT)                                                                                                  \
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(cfr_iter_d2v2_kernel<real, HC, GT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-#define CFRB_CFG(HC) CFRB_CFG1(HC, 32) CFRB_CFG1(HC, 64) CFRB_CFG1(HC, 128)
-  CFRB_CFG(0) CFRB_CFG(4) CFRB_CFG(5) CFRB_CFG(6) CFRB_CFG(9) CFRB_CFG(16)
-#undef CFRB_CFG
-#undef CFRB_CFG1
-  return e;
-}
-template <typename real>
-int cfr_d2v2_smem_bytes(int Nmax, int H, int Hout, int Lmax, int Tmax, int n1max, int stride) {
-  return D2v2Layout((int)sizeof(real), Nmax, H, Hout, Lmax, Tmax, n1max, stride).bytes;
-}
-template <typename real>
-void cfr_launch_iter_d2v2(const CfrDev<real>& p, int blocks, int threads, size_t smem, cudaStream_t st, int iter, int do_b, int do_f, int n1max) {
-#define CFRB_CALL(HC)                                                                                                      \
-  do {                                                                                                                     \
-    if (threads == 128) launch_pdl(cfr_iter_d2v2_kernel<real, HC, 128>, blocks, 128, smem, st, p, iter, do_b, do_f, n1max);  \
-    else if (threads == 64) launch_pdl(cfr_iter_d2v2_kernel<real, HC, 64>, blocks, 64, smem, st, p, iter, do_b, do_f, n1max); \
-    else launch_pdl(cfr_iter_d2v2_kernel<real, HC, 32>, blocks, 32, smem, st, p, iter, do_b, do_f, n1max);                  \
-  } while (0)
-  CFRB_DISPATCH_H(p.H, CFRB_CALL)
-#undef CFRB_CALL
-}
-
 // div_by_rcp against IEEE division on pseudo-random operands: quotient mantissas spread over [1, 2), including operands whose
 // quotient lies within a few ulp of a power of two and denominators with all-ones / all-zeros low mantissa bits.
 __global__ void div_check_kernel(unsigned long long seed, unsigned long long* mismatches) {
@@ -170,9 +142,6 @@ void div_check_launch(unsigned long long seed, int blocks, unsigned long long* m
   template void cfr_launch_iter<real>(const CfrDev<real>&, int, int, int, size_t, cudaStream_t, int, int, int, int);             \
   template cudaError_t cfr_configure_d2<real>(int);                                                                        \
   template void cfr_launch_iter_d2<real>(const CfrDev<real>&, int, int, size_t, cudaStream_t, int, int, int, int);                \
-  template cudaError_t cfr_configure_d2v2<real>(int);                                                                      \
-  template int cfr_d2v2_smem_bytes<real>(int, int, int, int, int, int, int);                                                \
-  template void cfr_launch_iter_d2v2<real>(const CfrDev<real>&, int, int, size_t, cudaStream_t, int, int, int, int);             \
   template void sp_launch_begin<real>(const SpDev&, real*, cudaStream_t);                                                  \
   template void sp_launch_finish<real>(const SpDev&, const real*, const real*, float*, float*, cudaStream_t);
 CFRB_INSTANTIATE(float)

@@ -502,13 +502,6 @@ __device__ __forceinline__ D2Tmpl d2_tmpl_view(const unsigned char* b, int HF) {
   (void)HF;
   return t;
 }
-__device__ __forceinline__ D2Levels d2_levels(const int* __restrict__ level_begin, const TemplateDev& t) {   // from the int arrays (cfr_d2v2.cuh)
-  D2Levels L;
-  L.n1b = level_begin[t.level_off + 1];
-  L.n1e = t.levels >= 2 ? level_begin[t.level_off + 2] : L.n1b;
-  L.n2e = t.levels >= 3 ? level_begin[t.level_off + 3] : L.n1e;
-  return L;
-}
 __device__ __forceinline__ D2Levels d2_levels(const unsigned char* b) {
   D2Levels L;
   L.n1b = 1; L.n1e = b[4]; L.n2e = b[5];

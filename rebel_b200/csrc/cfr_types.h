@@ -104,12 +104,7 @@ template <typename real> void sp_launch_finish(const SpDev& p, const real* mu, c
 // rows [ids[i]] of a [*, width] fp32 matrix -> out[i]  (replay sampling)
 void rows_launch_gather(const float* src, int width, const int* ids, int n, float* out, cudaStream_t st);
 
-// Generation-2 depth <= 2 kernel (cfr_d2v2.cuh): one warp per CTA, inputs staged by cp.async.bulk.
-template <typename real> cudaError_t cfr_configure_d2v2(int smem_bytes);
-template <typename real> int cfr_d2v2_smem_bytes(int Nmax, int H, int Hout, int Lmax, int Tmax, int n1max, int stride);
-template <typename real> void cfr_launch_iter_d2v2(const CfrDev<real>& p, int blocks, int threads, size_t smem, cudaStream_t st, int iter,
-                                                   int do_b, int do_f, int n1max);
-// Development check of div_by_rcp (cfr_d2v2.cuh): n pseudo-random (x, b) pairs per call, returns the number of quotients that
+// Development check of div_by_rcp (cfr_kernels.cuh): n pseudo-random (x, b) pairs per call, returns the number of quotients that
 // differ from x / b in *mismatches (device pointer).
 void div_check_launch(unsigned long long seed, int blocks, unsigned long long* mismatches, cudaStream_t st);
 

@@ -1,22 +1,11 @@
-// Tensor-core evaluation of the leaf value net (Net2: Linear -> LayerNorm -> GELU -> Linear -> LayerNorm -> GELU -> Linear,
-// cfvpy/models.py:64-94) for all pseudo-leaf query rows of a wave — the one dense contraction of the CFR hot path and,
-// at 148k FLOP per row, its dominant cost.  Blackwell-native: tcgen05.mma (kind::f16, fp16 operands, fp32 accumulation in
-// TMEM), weights resident in shared memory for the lifetime of a persistent CTA, activations never leave the SM:
+// Primitives and the weight-blob layout of the tcgen05 value net (the kernel: leaf_mlp_tc3.cuh).  The net is Net2: Linear ->
+// LayerNorm -> GELU -> Linear -> LayerNorm -> GELU -> Linear (cfvpy/models.py:64-94), evaluated with tcgen05.mma (kind::f16, fp16
+// operands, fp32 accumulation in TMEM) on 128-row tiles of pseudo-leaf query rows.
 //
-//   X tile [128 x Kp] fp16 (smem, UMMA K-major core-matrix order, written in that order by the CFR forward kernel)
-//     --tcgen05.mma SS-->  D1 [128 x 256] fp32 in TMEM cols [0,256)
-//     --epilogue (tcgen05.ld, +bias, LayerNorm, GELU, ->fp16, tcgen05.st)-->  A2 [128 x 256] fp16 in TMEM cols [256,384)
-//     --tcgen05.mma TS (A from TMEM, W2 from smem)-->  D2 in TMEM cols [0,256)   (reuses D1's columns)
-//     --epilogue-->  A3 in TMEM cols [256,384)
-//     --tcgen05.mma TS (N = 16)-->  D3 [128 x 16] in TMEM cols [384,400)  --epilogue (+bias)-->  out[rows][H] fp32
-//
-// Warp roles (544 threads): warps 0-15 = epilogue — warp w owns TMEM lanes 32*(w&3).. (one row per thread) and the column
-// quarter (w>>2), so a thread keeps its 64 accumulators in registers, reads TMEM once per layer and exchanges its LayerNorm
-// partial sums with the three partner warps through shared memory; warp 16 = TMEM allocator + single-thread MMA issuer.
+// Shapes shared by the host and the kernel: 544 threads per CTA, warps 0-15 = epilogue (warp w owns TMEM lanes 32*(w&3).., one
+// row per thread, and the column quarter (w>>2) of the 256 hidden features), warp 16 = TMEM allocator + single-thread MMA issuer.
 // The biases ride on the tensor cores: layer 1 through a constant-1 query column (written by the CFR kernel) against a bias
-// column in W1, layer 2 through one extra K=16 MMA of a constant "ones" tile against a bias tile.
-// mbarriers: x (query tile staged), d1/d2/d3 (accumulator ready, via tcgen05.commit), a2/a3 (A operand ready).
-// Each barrier completes exactly once per tile, so one parity bit per tile iteration serves all of them.
+// column in W1, layer 2 through one extra K=16 MMA of a constant "ones" tile against a bias tile; both live in the blob.
 #pragma once
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
@@ -33,12 +22,12 @@ constexpr int kColsPerThread = kHid / kParts;   // 64
 constexpr int kEpiThreads = 128 * kParts;    // 16 epilogue warps
 constexpr int kSubChunks = 4;                // A-operand hand-over granularity: 16 features per thread
 constexpr int kThreads = kEpiThreads + 32;   // + allocator / MMA-issuer warp
-constexpr uint32_t kColD = 0, kColA = 256, kColD3 = 384, kTmemCols = 512;
+constexpr uint32_t kColD = 0, kTmemCols = 512;
 
-// ---- shared-memory / weight-blob layout (bytes).  The blob in global memory has exactly the smem layout up to kOffX.
+// ---- weight-blob layout (bytes).  The blob in global memory has exactly the shared-memory layout up to off_x.
 struct BlobLayout {
   int Kp;            // padded query width (multiple of 16, with at least one spare column for the constant 1)
-  int off_w1, off_w2, off_w3, off_ones, off_bias2, off_ln1, off_ln2, off_b3, blob_bytes, off_x, off_part, off_bar, smem_bytes;
+  int off_w1, off_w2, off_w3, off_ones, off_bias2, off_ln1, off_ln2, off_b3, blob_bytes, off_x;
   __host__ __device__ explicit BlobLayout(int kp) : Kp(kp) {
     off_w1 = 0;                               // [256 x Kp]  fp16, column Q holds bias 1
     off_w2 = off_w1 + kHid * kp * 2;          // [256 x 256] fp16
@@ -49,10 +38,7 @@ struct BlobLayout {
     off_ln2 = off_ln1 + kHid * 8;
     off_b3 = off_ln2 + kHid * 8;
     blob_bytes = off_b3 + kNout * 4;
-    off_x = (blob_bytes + 127) / 128 * 128;
-    off_part = off_x + kTileM * kp * 2;       // LayerNorm partial sums: [2 layers][kParts][128 rows] float2
-    off_bar = off_part + 2 * kParts * kTileM * 8;
-    smem_bytes = off_bar + 192;            // 16 mbarriers + TMEM base slot
+    off_x = (blob_bytes + 127) / 128 * 128;   // first byte of shared memory after the weights (Tc3Layout)
   }
 };
 
@@ -80,7 +66,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
       "bra WAIT_LOOP;\n\t"
       "WAIT_DONE:\n\t}" ::"r"(bar), "r"(parity) : "memory");
 }
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_commit(uint32_t bar) {
@@ -130,13 +115,6 @@ __device__ __forceinline__ constexpr uint32_t make_idesc(int M, int N) {
         "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])                          \
       : "r"(taddr))
 
-#define CFRB_TMEM_ST16(taddr, v)                                                                                          \
-  asm volatile(                                                                                                           \
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr), \
-      "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),       \
-      "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])                                              \
-      : "memory")
-
 #define CFRB_TMEM_ST8(taddr, v)                                                                                           \
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), "r"(v[0]), "r"(v[1]),  \
                "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])                                           \
@@ -178,107 +156,7 @@ __device__ __forceinline__ float gelu_tc(float y) {
   return y * r;
 }
 
-// The same function on a packed pair of fp16 values: y * Phi(y) = hy + hy * tanh(y (c0 + c1 y^2 + c2 y^4)), hy = y / 2, with
-// HFMA2 arithmetic and one tanh.approx.f16x2 per pair (a quarter of the MUFU work and ~40 % of the instructions of gelu_tc).
-// The fp16 evaluation adds ~1.8e-4 rms (N(0,1) inputs) to the 1.4e-4 rms of rounding the activation to fp16 at all.
-__device__ __forceinline__ uint32_t gelu_tc_x2(float y0, float y1) {
-  const __half2 y = __floats2half2_rn(y0, y1);
-  const __half2 y2 = __hmin2(__hmul2(y, y), __float2half2_rn(52.f));
-  const __half2 p = __hfma2(y2, __hfma2(y2, __float2half2_rn(-3.5151e-4f), __float2half2_rn(3.70057e-2f)), __float2half2_rn(0.797496f));
-  const __half2 u = __hmul2(y, p);
-  uint32_t t;
-  asm("tanh.approx.f16x2 %0, %1;" : "=r"(t) : "r"(*reinterpret_cast<const uint32_t*>(&u)));
-  const __half2 hy = __hmul2(y, __float2half2_rn(0.5f));
-  const __half2 g = __hfma2(hy, *reinterpret_cast<const __half2*>(&t), hy);
-  return *reinterpret_cast<const uint32_t*>(&g);
-}
-
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
-
-// LayerNorm(eps 1e-5) + GELU of this thread's quarter row: 64 fp32 accumulators (TMEM lane = row, columns part*64..),
-// bias already added by the tensor cores, kept in registers; the four threads of a row exchange (sum, sum of squares)
-// through `part`.  Result as fp16 into the A-operand columns.  ln: float2 {gamma, beta} per feature in smem (broadcast reads).
-template <bool kDebug, bool kGeluX2>
-__device__ __forceinline__ void epilogue_ln_gelu(uint32_t tmem_row, int part_id, int row, const float2* __restrict__ ln, float2* part,
-                                                 uint32_t bar_a0, uint32_t bar_dfree, float* dbg_row, long long* tr) {
-  uint32_t xr[kColsPerThread];
-  float sum, sumsq;
-  {
-    // the second half of the quarter row is still arriving from TMEM while the first half is summed
-    uint32_t* lo = xr; uint32_t* hi = xr + 32;
-    CFRB_TMEM_LD32(tmem_row + kColD + part_id * kColsPerThread, lo);
-    tmem_wait_ld();
-    CFRB_TMEM_LD32(tmem_row + kColD + part_id * kColsPerThread + 32, hi);
-    if (kDebug && tr) tr[0] = clock64();
-    // two independent accumulator pairs: 2 x 2 interleaved chains of 16 packed adds / fmas instead of one chain of 32
-    f32x2 s2[2], q2[2];
-#pragma unroll
-    for (int u = 0; u < 2; ++u) { s2[u] = pack2(0.f, 0.f); q2[u] = pack2(0.f, 0.f); }
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {
-      if (half == 1) tmem_wait_ld();
-#pragma unroll
-      for (int i = half * 32; i < half * 32 + 32; i += 2) {
-        if (kDebug && dbg_row) {
-          dbg_row[part_id * kColsPerThread + i] = __uint_as_float(xr[i]);
-          dbg_row[part_id * kColsPerThread + i + 1] = __uint_as_float(xr[i + 1]);
-        }
-        const f32x2 x2 = pack2(__uint_as_float(xr[i]), __uint_as_float(xr[i + 1]));
-        s2[(i >> 1) & 1] = add2(s2[(i >> 1) & 1], x2);
-        q2[(i >> 1) & 1] = fma2(x2, x2, q2[(i >> 1) & 1]);
-      }
-    }
-    const f32x2 st = add2(s2[0], s2[1]), qt = add2(q2[0], q2[1]);
-    float a0, a1, b0, b1;
-    unpack2(st, a0, a1); unpack2(qt, b0, b1);
-    sum = a0 + a1; sumsq = b0 + b1;
-  }
-  part[part_id * kTileM + row] = make_float2(sum, sumsq);
-  if (kDebug && tr) tr[1] = clock64();
-  named_bar_sync(1, kEpiThreads);
-  // every accumulator of the tile now lives in registers: the D columns may be overwritten (next tile's layer 1)
-  if (bar_dfree) {
-    tc_fence_before();
-    mbar_arrive(bar_dfree);
-  }
-  if (kDebug && tr) tr[2] = clock64();
-  sum = 0.f; sumsq = 0.f;
-#pragma unroll
-  for (int p = 0; p < kParts; ++p) {          // fixed order: all four threads of a row get bit-identical statistics
-    const float2 o = part[p * kTileM + row];
-    sum += o.x; sumsq += o.y;
-  }
-  const float mean = sum * (1.f / kHid);
-  const float var = fmaxf(sumsq * (1.f / kHid) - mean * mean, 0.f);
-  const float rstd = rsqrtf(var + 1e-5f);
-  const float shift = -mean * rstd;
-  const f32x2 rstd2 = pack2(rstd, rstd), shift2 = pack2(shift, shift);
-  // Four sub-chunks of 16 features: sub-chunk s of column quarter q is K-step 4q+s of the next layer's MMA, so after the
-  // s-th arrival of all epilogue threads the issuer can run K-steps {s, 4+s, 8+s, 12+s} while the rest is still being
-  // normalised (only the last quarter of the MMA stays exposed).
-#pragma unroll
-  for (int c = 0; c < kSubChunks; ++c) {
-    uint32_t pk[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const int j = c * 16 + 2 * i;
-      const float4 pp = *reinterpret_cast<const float4*>(ln + part_id * kColsPerThread + j);   // {gamma_j, gamma_j+1, beta_j, beta_j+1}
-      float y0, y1;
-      unpack2(fma2(fma2(pack2(__uint_as_float(xr[j]), __uint_as_float(xr[j + 1])), rstd2, shift2), pack2(pp.x, pp.y), pack2(pp.z, pp.w)), y0, y1);
-      if (kGeluX2) {
-        pk[i] = gelu_tc_x2(y0, y1);
-      } else {
-        const __half2 h = __floats2half2_rn(gelu_tc(y0), gelu_tc(y1));
-        pk[i] = *reinterpret_cast<const uint32_t*>(&h);
-      }
-    }
-    CFRB_TMEM_ST8(tmem_row + kColA + part_id * (kColsPerThread / 2) + c * 8, pk);
-    tmem_wait_st();
-    tc_fence_before();
-    mbar_arrive(bar_a0 + 8 * c);
-  }
-  if (kDebug && tr) tr[3] = clock64();
-}
 
 struct TcArgs {
   const uint8_t* blob;      // weights in smem layout (BlobLayout)
@@ -288,195 +166,9 @@ struct TcArgs {
   int Kp, H, Hout;
   float* dbg_d1;            // optional [128][256] raw layer-1 accumulators of tile 0
   float* dbg_d2;            // optional [128][256] raw layer-2 accumulators of tile 0
-  long long* trace;         // optional (debug build only): SM clock stamps of CTA 0, [2048]: epilogue thread 0 at
-                            // [iter*16 + e], MMA thread at [1024 + iter*8 + m]
+  long long* trace;         // optional (debug launch only): SM clock stamps of CTA 0, [2048]: epilogue thread 0 at
+                            // [phase*8 + e], MMA issuer at [1024 + phase*4 + m]
 };
-
-#define CFRB_TRACE(slot)                                                      \
-  do {                                                                        \
-    if (kDebug && a.trace && blockIdx.x == 0 && it_no < 60) a.trace[slot] = clock64(); \
-  } while (0)
-
-template <bool kDebug, bool kGeluX2>
-__global__ void __launch_bounds__(kThreads, 1) leaf_mlp_tc_kernel(TcArgs a) {
-  constexpr int kMmaWarp = kEpiThreads / 32;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  const BlobLayout L(a.Kp);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int rows = *a.rows_ptr;
-  const int ntiles = (rows + kTileM - 1) / kTileM;
-  if ((int)blockIdx.x >= ntiles) return;
-
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L.off_bar);
-  // bars: 0 x, 1 d1, 2 d2, 3 d3, 4 dfree, 8..11 a2[sub-chunk], 12..15 a3[sub-chunk]
-  const uint32_t bar_x = smem_u32(bars + 0), bar_d1 = smem_u32(bars + 1), bar_d2 = smem_u32(bars + 2), bar_d3 = smem_u32(bars + 3),
-                 bar_dfree = smem_u32(bars + 4), bar_a2 = smem_u32(bars + 8), bar_a3 = smem_u32(bars + 12);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 16);
-
-  // ---- one-time setup: weights -> smem, barriers, TMEM
-  {
-    const int4* src = reinterpret_cast<const int4*>(a.blob);
-    int4* dst = reinterpret_cast<int4*>(smem);
-    for (int i = tid; i < L.blob_bytes / 16; i += kThreads) dst[i] = __ldg(src + i);
-  }
-  if (tid == 0) {
-    mbar_init(bar_x, kEpiThreads); mbar_init(bar_d1, 1); mbar_init(bar_d2, 1); mbar_init(bar_d3, 1);
-    mbar_init(bar_dfree, kEpiThreads);
-    for (int c = 0; c < kSubChunks; ++c) { mbar_init(bar_a2 + 8 * c, kEpiThreads); mbar_init(bar_a3 + 8 * c, kEpiThreads); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == kMmaWarp) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  fence_proxy_async_smem();          // generic-proxy weight stores -> visible to the tensor-core (async) proxy
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  // Everything above (weights -> shared memory, barriers, TMEM) is independent of the CFR kernel that precedes this launch:
-  // with programmatic dependent launch it runs while that kernel drains.  From here on its query tiles are read.
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  asm volatile("griddepcontrol.launch_dependents;");
-
-  const uint32_t sx = smem_u32(smem + L.off_x), sw1 = smem_u32(smem + L.off_w1), sw2 = smem_u32(smem + L.off_w2),
-                 sw3 = smem_u32(smem + L.off_w3), sones = smem_u32(smem + L.off_ones), sbias2 = smem_u32(smem + L.off_bias2);
-  const int x_tile_int4 = kTileM * a.Kp * 2 / 16;
-
-  if (warp == kMmaWarp) {
-    // ===================== MMA issuer (one thread) =====================
-    if (lane == 0) {
-      const uint32_t idesc256 = make_idesc(kTileM, kHid), idesc16 = make_idesc(kTileM, kNout);
-      const uint32_t lbo_x = (kTileM / 8) * 128, lbo_w = (kHid / 8) * 128, lbo_w3 = (kNout / 8) * 128;
-      // Layer 1 of tile n+1 is issued inside iteration n, as soon as the epilogue warps hold tile n's layer-2 accumulators in
-      // registers (dfree) — the D columns are free then and the tensor pipe would otherwise idle through epilogue 2.
-      mbar_wait(bar_x, 0);
-      tc_fence_after();
-      for (int k = 0; k < a.Kp / 16; ++k)
-        mma_ss(tmem_base + kColD, make_desc(sx + k * 2 * lbo_x, lbo_x, 128), make_desc(sw1 + k * 2 * lbo_w, lbo_w, 128), idesc256, k > 0);
-      tc_commit(bar_d1);
-      uint32_t parity = 0;
-      int it_no = 0;
-      for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, parity ^= 1, ++it_no) {
-        // layer 2: D2 = ones * bias2^T + A2 * W2^T  (A from TMEM: 16 fp16 = 8 columns per K step), K-steps in the order the
-        // epilogue hands them over
-        for (int c = 0; c < kSubChunks; ++c) {
-          mbar_wait(bar_a2 + 8 * c, parity);
-          tc_fence_after();
-          if (c == 0) {
-            CFRB_TRACE(1024 + it_no * 8 + 2);
-            mma_ss(tmem_base + kColD, make_desc(sones, lbo_x, 128), make_desc(sbias2, lbo_w, 128), idesc256, 0);
-          }
-          for (int q = 0; q < kParts; ++q) {
-            const int k = q * kSubChunks + c;
-            mma_ts(tmem_base + kColD, tmem_base + kColA + k * 8, make_desc(sw2 + k * 2 * lbo_w, lbo_w, 128), idesc256, 1);
-          }
-        }
-        tc_commit(bar_d2);
-        CFRB_TRACE(1024 + it_no * 8 + 3);
-        // layer 1 of the next tile
-        if (tile + (int)gridDim.x < ntiles) {
-          mbar_wait(bar_dfree, parity);
-          mbar_wait(bar_x, parity ^ 1);
-          tc_fence_after();
-          CFRB_TRACE(1024 + it_no * 8 + 0);
-          for (int k = 0; k < a.Kp / 16; ++k)
-            mma_ss(tmem_base + kColD, make_desc(sx + k * 2 * lbo_x, lbo_x, 128), make_desc(sw1 + k * 2 * lbo_w, lbo_w, 128), idesc256, k > 0);
-          tc_commit(bar_d1);
-          CFRB_TRACE(1024 + it_no * 8 + 1);
-        }
-        // layer 3: D3 = A3 * W3^T  (N = 16)
-        for (int c = 0; c < kSubChunks; ++c) {
-          mbar_wait(bar_a3 + 8 * c, parity);
-          tc_fence_after();
-          if (c == 0) CFRB_TRACE(1024 + it_no * 8 + 4);
-          for (int q = 0; q < kParts; ++q) {
-            const int k = q * kSubChunks + c;
-            mma_ts(tmem_base + kColD3, tmem_base + kColA + k * 8, make_desc(sw3 + k * 2 * lbo_w3, lbo_w3, 128), idesc16, (c | q) != 0);
-          }
-        }
-        tc_commit(bar_d3);
-        CFRB_TRACE(1024 + it_no * 8 + 5);
-      }
-    }
-  } else {
-    // ===================== epilogue warps: thread == (row, column quarter) =====================
-    const int quad = warp & 3, part_id = warp >> 2;
-    const int row_in_tile = quad * 32 + lane;                      // 0..127 == TMEM lane
-    const uint32_t tmem_row = tmem_base + ((uint32_t)(quad * 32) << 16);
-    const float2* ln1 = reinterpret_cast<const float2*>(smem + L.off_ln1);
-    const float2* ln2 = reinterpret_cast<const float2*>(smem + L.off_ln2);
-    const float* b3 = reinterpret_cast<const float*>(smem + L.off_b3);
-    float2* part1 = reinterpret_cast<float2*>(smem + L.off_part);
-    float2* part2 = part1 + kParts * kTileM;
-    int4* xdst = reinterpret_cast<int4*>(smem + L.off_x);
-    const int x_items = x_tile_int4;                               // 512 or 768 int4 per tile: <= 2 per thread
-    int4 xr0, xr1;
-    {
-      const int4* xsrc = reinterpret_cast<const int4*>(a.Xh) + (size_t)blockIdx.x * x_tile_int4;
-      for (int i = tid; i < x_items; i += kEpiThreads) xdst[i] = __ldg(xsrc + i);
-      fence_proxy_async_smem();
-      mbar_arrive(bar_x);
-    }
-    uint32_t parity = 0;
-    int it_no = tid == 0 ? 0 : 1 << 20;     // only thread 0 leaves trace stamps
-    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, parity ^= 1, ++it_no) {
-      const int next = tile + gridDim.x;
-      const bool dbg = (tile == 0);
-      // ---- layer-1 accumulators ready; the query tile in smem is free again -> start fetching the next one
-      mbar_wait(bar_d1, parity);
-      tc_fence_after();
-      CFRB_TRACE(it_no * 16 + 0);
-      if (next < ntiles) {
-        const int4* xsrc = reinterpret_cast<const int4*>(a.Xh) + (size_t)next * x_tile_int4;
-        xr0 = __ldg(xsrc + tid);
-        if (tid + kEpiThreads < x_items) xr1 = __ldg(xsrc + tid + kEpiThreads);
-      }
-      epilogue_ln_gelu<kDebug, kGeluX2>(tmem_row, part_id, row_in_tile, ln1, part1, bar_a2, 0u, (dbg && a.dbg_d1) ? a.dbg_d1 + row_in_tile * kHid : nullptr,
-                                        (kDebug && a.trace && blockIdx.x == 0 && it_no < 60) ? a.trace + it_no * 16 + 7 : nullptr);
-      CFRB_TRACE(it_no * 16 + 1);
-      if (next < ntiles) {
-        xdst[tid] = xr0;
-        if (tid + kEpiThreads < x_items) xdst[tid + kEpiThreads] = xr1;
-        fence_proxy_async_smem();
-        mbar_arrive(bar_x);
-      }
-      // ---- layer 2
-      CFRB_TRACE(it_no * 16 + 2);
-      mbar_wait(bar_d2, parity);
-      tc_fence_after();
-      CFRB_TRACE(it_no * 16 + 3);
-      epilogue_ln_gelu<kDebug, kGeluX2>(tmem_row, part_id, row_in_tile, ln2, part2, bar_a3, next < ntiles ? bar_dfree : 0u,
-                                        (dbg && a.dbg_d2) ? a.dbg_d2 + row_in_tile * kHid : nullptr,
-                                        (kDebug && a.trace && blockIdx.x == 0 && it_no < 60) ? a.trace + it_no * 16 + 11 : nullptr);
-      CFRB_TRACE(it_no * 16 + 4);
-      // ---- layer 3: raw net outputs (the CFR backward kernel multiplies by the opponent-reach scaler)
-      mbar_wait(bar_d3, parity);
-      tc_fence_after();
-      CFRB_TRACE(it_no * 16 + 5);
-      if (part_id == 0) {
-        uint32_t v[16];
-        CFRB_TMEM_LD16(tmem_row + kColD3, v);
-        tmem_wait_ld();
-        const int row = tile * kTileM + row_in_tile;
-        if (row < rows) {
-          float* o = a.out + (size_t)row * a.Hout;
-#pragma unroll
-          for (int h = 0; h < kNout; ++h) if (h < a.H) o[h] = __uint_as_float(v[h]) + b3[h];
-        }
-      }
-      CFRB_TRACE(it_no * 16 + 6);
-      tc_fence_before();   // order this tile's TMEM reads before the next tile's MMAs (via the a2/a3/x arrivals that follow)
-    }
-  }
-  // ---- teardown
-  tc_fence_before();
-  __syncthreads();
-  if (warp == kMmaWarp) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
-  }
-}
 
 }  // namespace tc
 }  // namespace cfrb

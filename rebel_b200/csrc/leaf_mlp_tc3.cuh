@@ -1,10 +1,11 @@
-// Tensor-core evaluation of the leaf value net, generation 3: the kernel of leaf_mlp_tc.cuh (tcgen05.mma kind::f16, fp32
-// accumulation in TMEM, weights resident in shared memory, activations fed back to the tensor cores from TMEM) re-scheduled so
-// that the epilogue warps never wait for the tensor pipe, with a cheaper epilogue, and with every global->shared transfer done
-// by the bulk-copy engine (cp.async.bulk + mbarrier complete_tx; SASS: UBLKCP).
+// Tensor-core evaluation of the leaf value net (Net2: Linear -> LayerNorm -> GELU -> Linear -> LayerNorm -> GELU -> Linear,
+// cfvpy/models.py:64-94) for all pseudo-leaf query rows of a wave, generation 3: tcgen05.mma kind::f16 with fp32 accumulation in
+// TMEM, weights resident in shared memory, activations fed back to the tensor cores from TMEM, scheduled so that the epilogue
+// warps never wait for the tensor pipe, and with every global->shared transfer done by the bulk-copy engine (cp.async.bulk +
+// mbarrier complete_tx; SASS: UBLKCP).  Primitives and the weight-blob layout: leaf_mlp_tc.cuh.
 //
-// What changed against generation 1 (measured there: 11 100 cycles per 128-row tile = 2 x 4 550 epilogue + 1 340 exposed MMA
-// tails + 500 output; tensor pipe 26 % busy):
+// What changed against generation 1 (a one-tile kernel, removed after commit 76e7204; measured there: 11 100 cycles per 128-row
+// tile = 2 x 4 550 epilogue + 1 340 exposed MMA tails + 500 output; tensor pipe 26 % busy):
 //
 //  1. TWO TILES IN FLIGHT, ONE ACCUMULATOR REGION.  TMEM = D [0,256) | A0 [256,384) | A1 [384,512): a single fp32 accumulator
 //     region shared by both tiles and one fp16 A-operand region per tile.  The 16 epilogue warps run the phases
@@ -20,9 +21,9 @@
 //     (W'[j][k] = W[j][k] - mean_j W[j][k]), so sum_j y_j = 0 by construction and LayerNorm needs only sum_j y_j^2: the
 //     running-sum chain, the mean and the shift disappear from the epilogue (two-pass-quality variance for free).
 //  3. HALVED GELU ARGUMENT.  The affine produces hy = y / 2 directly (gamma / 2 and beta / 2 are stored), the tanh polynomial is
-//     rescaled to hy, and GELU(y) = hy + hy * tanh(.): one multiply fewer per pair than before.  Default evaluation: packed
-//     f32x2 FMAs + tanh.approx.f32, rounded to fp16 once (gelu_hy_t32); the packed-fp16 evaluation (gelu_hy_x2) is 6 % faster
-//     but inherits the truncation of tanh.approx.f16x2 and is kept as a measurement option only.
+//     rescaled to hy, and GELU(y) = hy + hy * tanh(.): one multiply fewer per pair than before.  Evaluated with packed
+//     f32x2 FMAs + tanh.approx.f32, rounded to fp16 once (gelu_hy_t32).  A packed-fp16 evaluation (gelu_hy_x2, now only in the
+//     GELU table of cfrb_api.cu) was 6 % faster but inherits the truncation of tanh.approx.f16x2; it was removed after 76e7204.
 //  4. One mbarrier arrival per WARP (lane 0 after __syncwarp) instead of per thread, one A-operand hand-over per phase instead of
 //     four, LayerNorm partial sums exchanged between the four warps of a row quadrant only (named barrier of 128 threads).
 //  5. Weights (once per CTA) and query tiles (double-buffered, issued two tiles ahead by the MMA warp) arrive by cp.async.bulk.
@@ -61,23 +62,13 @@ __device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) {
   return r;
 }
 
-// GELU(y) for a packed pair given hy = y / 2:  hy + hy * tanh(hy (c0 + c1 hy^2 + c2 hy^4)), the coefficients of gelu_tc_x2
-// rescaled to hy (c0' = 2 c0, c1' = 8 c1, c2' = 32 c2) and the clamp y^2 <= 52 as hy^2 <= 13.
-__device__ __forceinline__ uint32_t gelu_hy_x2(float hy0, float hy1) {
-  const __half2 hy = __floats2half2_rn(hy0, hy1);
-  const __half2 s = __hmin2(__hmul2(hy, hy), __float2half2_rn(13.f));
-  const __half2 p = __hfma2(s, __hfma2(s, __float2half2_rn(-1.124832e-2f), __float2half2_rn(2.960456e-1f)), __float2half2_rn(1.594992f));
-  const __half2 u = __hmul2(hy, p);
-  uint32_t t;
-  asm("tanh.approx.f16x2 %0, %1;" : "=r"(t) : "r"(*reinterpret_cast<const uint32_t*>(&u)));
-  const __half2 g = __hfma2(hy, *reinterpret_cast<const __half2*>(&t), hy);
-  return *reinterpret_cast<const uint32_t*>(&g);
-}
-
-// The same function with fp32 arithmetic (packed f32x2 FMAs, tanh.approx.f32) and ONE rounding to fp16 at the end.  Measured
-// on B200 (profiles/r2_gelu_table.log): tanh.approx.f16x2 truncates towards zero (mean error -2.4e-4 sign(u) on 0.25 <= |u| < 4, one
-// fp16 ulp at most), which gives gelu_hy_x2 a coherent negative bias of 1.6e-4 .. 3.9e-4 on every activation with |y| > 0.5; the
-// data-generation statistics of the self-play loop respond to that bias (tests/test_rela_module.py P5), not to the rounding noise.
+// GELU(y) for a packed pair given hy = y / 2:  hy + hy * tanh(hy (c0 + c1 hy^2 + c2 hy^4)), the fit
+// tanh(y (0.797496 + 3.70057e-2 y^2 - 3.5151e-4 y^4)) rescaled to hy (c0 = 2 x, c1 = 8 x, c2 = 32 x) and the clamp y^2 <= 52 as
+// hy^2 <= 13.  fp32 arithmetic (packed f32x2 FMAs, tanh.approx.f32) with ONE rounding to fp16 at the end.  Not fp16: measured on
+// B200 (profiles/r2_gelu_table.log), tanh.approx.f16x2 truncates towards zero (mean error -2.4e-4 sign(u) on 0.25 <= |u| < 4, one
+// fp16 ulp at most), which gives the packed-fp16 evaluation (gelu_hy_x2, cfrb_api.cu) a coherent negative bias of 1.6e-4 ..
+// 3.9e-4 on every activation with |y| > 0.5; the data-generation statistics of the self-play loop respond to that bias
+// (tests/test_rela_module.py P5), not to the rounding noise.
 __device__ __forceinline__ uint32_t gelu_hy_t32(float hy0, float hy1) {
   const f32x2 hy = pack2(hy0, hy1);
   float s0, s1;
@@ -98,9 +89,8 @@ __device__ __forceinline__ uint32_t gelu_hy_t32(float hy0, float hy1) {
     if (kDebug && a.trace && blockIdx.x == 0 && (slot) < 2048) a.trace[slot] = clock64(); \
   } while (0)
 
-// kGelu: 0 = fp32 logistic GELU (CFRB_NET_TC_F16); 1 = packed-half GELU, 2 = fp32 tanh GELU (both CFRB_NET_TC_F16X2: the LayerNorm
-// parameters in the blob are gamma / 2, beta / 2)
-// (CFRB_NET_TC_F16; gamma, beta).
+// kGelu: 0 = fp32 logistic GELU (CFRB_NET_TC_F16; the LayerNorm parameters in the blob are gamma, beta); 2 = fp32 tanh GELU
+// (CFRB_NET_TC_F16X2; gamma / 2, beta / 2).
 template <bool kDebug, int kGelu>
 __global__ void __launch_bounds__(kThreads, 1) leaf_mlp_tc3_kernel(TcArgs a) {
   constexpr int kMmaWarp = kEpiThreads / 32;
@@ -319,9 +309,7 @@ __global__ void __launch_bounds__(kThreads, 1) leaf_mlp_tc3_kernel(TcArgs a) {
           const float4 pp = *reinterpret_cast<const float4*>(ln + part_id * kColsPerThread + jj);   // {g_j, g_j+1, b_j, b_j+1} (x2: halved)
           float y0, y1;
           unpack2(fma2(mul2(pack2(__uint_as_float(xr[jj]), __uint_as_float(xr[jj + 1])), rstd2), pack2(pp.x, pp.y), pack2(pp.z, pp.w)), y0, y1);
-          if (kGelu == 1) {
-            pk[i] = gelu_hy_x2(y0, y1);
-          } else if (kGelu == 2) {
+          if (kGelu == 2) {
             pk[i] = gelu_hy_t32(y0, y1);
           } else {
             const __half2 h = __floats2half2_rn(gelu_tc(y0), gelu_tc(y1));

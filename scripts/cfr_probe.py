@@ -1,4 +1,4 @@
-"""CFR kernel time (zero net: the iteration is the CFR kernel alone) for root waves and for self-play waves, both kernel generations."""
+"""CFR kernel time (zero net: the iteration is the CFR kernel alone) for root waves and for self-play waves."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -12,11 +12,11 @@ S.begin(np.full(K, -1, np.int32), np.zeros(K, np.int32), b)
 for _ in range(3):
     S.reset(); S.run(256); S.sync()
 tot, _ = S.last_run_ms()
-print("gen", os.environ.get("CFRB_D2_GEN", "1.5") + "/" + os.environ.get("CFRB_D2V2_THREADS", "32"), "root wave: CFR us per iteration", tot / 256 * 1e3, flush=True)
+print("root wave: CFR us per iteration", tot / 256 * 1e3, flush=True)
 S.selfplay_create(np.arange(K, dtype=np.uint32) * 1000000 + 7)
 for _ in range(8):
     S.selfplay_wave()
 S.sync()
 S.selfplay_wave(); S.sync()
 tot, _ = S.last_run_ms()
-print("gen", os.environ.get("CFRB_D2_GEN", "1.5") + "/" + os.environ.get("CFRB_D2V2_THREADS", "32"), "self-play wave: CFR us per iteration", tot / 1024 * 1e3, "rows", S.leaf_rows, flush=True)
+print("self-play wave: CFR us per iteration", tot / 1024 * 1e3, "rows", S.leaf_rows, flush=True)

@@ -106,12 +106,18 @@ CONFIGS = [("f64", "zero"), ("f64", "fp32"), ("f32", "zero"), ("f32", "fp32"), (
 NETS = lambda rb: {"zero": rb.NET_ZERO, "fp32": rb.NET_FP32, "tc": rb.NET_TC_F16, "tcx2": rb.NET_TC_F16X2}
 
 
-@pytest.mark.parametrize("D,F", SHAPES)
+@pytest.mark.parametrize("D,F", SHAPES + [(2, 4)])
 @pytest.mark.parametrize("state_name,net_name", CONFIGS)
 @pytest.mark.parametrize("max_depth", [2, 3])
-def test_teacher_forced_single_step(rb, port, net_weights, D, F, state_name, net_name, max_depth):
+def test_teacher_forced_single_step(rb, port, net_weights, monkeypatch, D, F, state_name, net_name, max_depth):
     if net_name in ("tc", "tcx2") and max_depth != 2:
         pytest.skip("tensor-core net is exercised on the data-generation depth")
+    if (D, F) == (2, 4):
+        # 16 hands on the generic CFR kernel, bit for bit: at depth 3 the scratch needs a CTA per subgame
+        # (cfr_iter_kernel<double, 256, 0>), at depth 2 CFRB_NO_D2=1 selects the 16-hand warp kernel (cfr_iter_kernel<double, 32, 16>)
+        if (state_name, net_name) != ("f64", "zero"):
+            pytest.skip("2x4f covers the generic kernel's 16-hand paths in the bit-exact configuration")
+        monkeypatch.setenv("CFRB_NO_D2", "1")
     A, H, Q = game_dims(D, F)
     state = {"f64": rb.STATE_F64, "f32": rb.STATE_F32}[state_name]
     net = NETS(rb)[net_name]
@@ -541,7 +547,7 @@ def test_snapshot_of_act_iteration_zero_needs_no_run(rb, port):
 
 
 def test_fast_division_is_correctly_rounded(rb):
-    """cfr_iter_d2v2_kernel obtains sigma = max(R, eps) / sum from the reciprocal of the sum (one true division per (node, hand))
+    """cfr_iter_d2_kernel obtains sigma = max(R, eps) / sum from the reciprocal of the sum (one true division per (node, hand))
     and two fused multiply-add correction steps instead of one IEEE division per action.  The quotients must be the correctly
     rounded ones — the bits `/` gives — or the solver would leave the reference's trajectory: 4.3e9 pseudo-random operand pairs
     (uniform mantissas, denominators next to 1 and 2, quotients within a few ulp of 1, the 1e-80 scale, small-integer multiples)."""
@@ -553,8 +559,8 @@ def test_fast_division_is_correctly_rounded(rb):
 
 def test_fast_gelu_is_unbiased(rb):
     """The value-net epilogue's fast GELU on EVERY fp16 input (cfrb_debug_gelu_table): the default fp32-tanh evaluation must be
-    as good as rounding the exact erf-GELU to fp16 — no systematic error.  The packed-fp16 evaluation (CFRB_X2_GELU=half) is
-    measured next to it: tanh.approx.f16x2 truncates towards zero, which biases every activation with |y| > 0.5 by -1.6e-4 ..
+    as good as rounding the exact erf-GELU to fp16 — no systematic error.  The packed-fp16 evaluation of the same formula (an
+    earlier epilogue, now only a table of cfrb_debug_gelu_table) is measured next to it: tanh.approx.f16x2 truncates towards zero, which biases every activation with |y| > 0.5 by -1.6e-4 ..
     -3.9e-4; in the self-play loop that coherent bias moved the generated distribution (P5) although its rms error (6.3e-4 of
     the net output against 5.0e-4) looked harmless."""
     from scipy.special import erf

@@ -449,7 +449,7 @@ def test_datagen_distribution_matches_reference(rela, golden, D, F, net_name, ne
     assert len(qk) >= 50000
     cnt, vsum, lsum = _last_action_stats(qk, vk, A, net)
     sets = {n: (g[f"count_{n}_{D}x{F}"].astype(np.float64), g[f"val_sum_{n}_{D}x{F}"], g[f"loss_sum_{n}_{D}x{F}"]) for n in ("a", "b")}
-    model = {"tc": "m1", "tcx2": "m1"}.get(net_name)       # m2 models the packed-half GELU (CFRB_X2_GELU=half) with an ideally rounded tanh
+    model = {"tc": "m1", "tcx2": "m1"}.get(net_name)       # m2 models the packed-half GELU (gelu_hy_x2) with an ideally rounded tanh
     if model is not None and f"count_{model}_{D}x{F}" in g.files:
         sets[model] = (g[f"count_{model}_{D}x{F}"].astype(np.float64), g[f"val_sum_{model}_{D}x{F}"], g[f"loss_sum_{model}_{D}x{F}"])
     big = np.ones(A + 1, bool)
